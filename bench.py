@@ -4,6 +4,7 @@
 Metric (BASELINE.json): candidate poses scored / s (+ loop-closure constraints / s).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C]
+                  [--dump-outputs DIR]
 
 --config 2 (default, the headline at every N): BASELINE config[1] — 2D
   FastCorrelativeScanMatcher MatchFullSubmap, 1081-beam synthetic scans vs a 1000x1000
@@ -24,6 +25,10 @@ Metric (BASELINE.json): candidate poses scored / s (+ loop-closure constraints /
 `e2e`    : the same work through the C ABI with HOST point clouds (H2D + D2H inside).
 `--impl reference`: the CPU oracle (restated reference path; the real reference does
 not build here, see DESIGN.md) on the host cores, same metric / workload.
+`--dump-outputs DIR` (config 2): after the timed steps, rank 0 writes the result records of
+  the last timed step (every rank's matches, job order) as DIR/<field>.npy, one file per
+  RESULT2D field.  The inputs are seeded, so two builds run with the same arguments can be
+  compared output for output.
 """
 import argparse
 import ctypes as C
@@ -134,6 +139,17 @@ def sample_clocks(local_rank, workload, min_seconds=1.5, min_iters=3):
     out["note"] = ("nvidia-smi -lms 100 while the same steps ran again right after the timed "
                    "region; no poller inside the timed legs")
     return out
+
+
+def dump_outputs(directory, records):
+    """One DIR/<field>.npy per field of `records`: float32 fields stay float32, the others
+    (float64 poses, int32 flags / indices / counts) are stored as float64, which holds
+    int32 exactly."""
+    os.makedirs(directory, exist_ok=True)
+    for name in records.dtype.names:
+        a = records[name]
+        np.save(os.path.join(directory, name + ".npy"),
+                a.astype(np.float32 if a.dtype == np.float32 else np.float64))
 
 
 def measured_peaks():
@@ -457,6 +473,8 @@ def bench_full_submap(args, D):
             coll_ms += st["collective_ms"]
             host_syncs = max(host_syncs, st["host_syncs"])
     launches = sm.kernel_launch_count() - launches0
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)   # the last timed step, all ranks' matches
     # per-step diagnostics: every rank's median / max step and the library-side split
     diag_v = D.gather_stats(step_s)
     elapsed = D.reduce([float(sum(step_s))], "MAX")[0]
@@ -785,7 +803,13 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=sorted(WORKLOADS))
     ap.add_argument("--scale", type=float, default=1.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's results as DIR/<field>.npy (config 2)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config != 2):
+        ap.error("--dump-outputs is implemented for the device path of --config 2")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)
